@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          # the CUDA wavefront backend
   python bench.py --impl reference --gpus N ...           # the CPU path (oracle), rank 0 only
+  python bench.py ... --dump-outputs DIR                  # also write the last timed step's outputs to DIR/*.npy
 
 A "step" is one frame: one pass of the hot path (raygen -> [closest-hit traversal -> shade ->
 any-hit traversal -> NEE resolve] x depth -> resolve/tonemap) over the whole image at the
@@ -275,6 +276,10 @@ def run_reference_arm(args):
             f += 1
             rays += st.num_rays
             ms += st.render_time
+    if args.dump_outputs:
+        # (a step keeps the workload's spp only where the frames fit CRT_BENCH_REF_BUDGET on this host, see above: with
+        # fewer, the outputs differ accordingly)
+        dump_outputs(args.dump_outputs, cpu.read_accum(), cpu.img, int(st.num_rays))
     value = rays / (ms * 1e3)
     cores = cpu_cores()
     line = {
@@ -443,6 +448,30 @@ def extra_workload_probe(workload_key: str):
         return {"error": f"{type(e).__name__}: {e}"[:300]}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, accum, img, num_rays: int, limit: int = DUMP_BYTES) -> None:
+    """--dump-outputs: what a caller of the render path holds after the last timed step, as .npy files, so that two builds
+    can be compared output for output. accum.npy: the accumulated radiance (float32, height x width x 3); img.npy: the
+    sRGB8 frame (`img`, one packed RGBA8 uint32 per pixel) as float32 R, G, B, A values 0..255 (height x width x 4);
+    num_rays.npy: the rays of that frame (float64). A frame whose two arrays exceed `limit` bytes is sampled at the same
+    seeded pixels every run: the arrays are then (n, 3) and (n, 4), and pixel_index.npy holds the row-major pixel indices
+    (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgba = img.view(np.uint8).reshape(img.shape + (4,)).astype(np.float32)
+    pixels = accum.shape[0] * accum.shape[1]
+    per_pixel = accum.itemsize * 3 + rgba.itemsize * 4
+    if pixels * per_pixel > limit:
+        n = (limit - 4096) // (per_pixel + 8)  # (4 KB for the .npy headers and num_rays.npy)
+        idx = np.sort(np.random.default_rng(0).choice(pixels, n, replace=False))
+        accum, rgba = accum.reshape(-1, 3)[idx], rgba.reshape(-1, 4)[idx]
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "accum.npy"), accum)
+    np.save(os.path.join(out_dir, "img.npy"), rgba)
+    np.save(os.path.join(out_dir, "num_rays.npy"), np.array([num_rays], np.float64))
+
+
 def emit(line: dict) -> None:
     """The contract is ONE JSON line on stdout. Libraries (NCCL prints its version banner) write
     to fd 1 too, so main() points fd 1 at stderr for the whole run and the result goes to the
@@ -474,9 +503,13 @@ def main():
     ap.add_argument("--profile-mode", action="store_true",
                     help="for runs under ncu: skip the instrumented counting pass and the CPU baseline")
     ap.add_argument("--repeats", type=int, default=5, help="repetitions of the K-step device-timed region (dispersion)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's framebuffers and ray count to DIR/<name>.npy")
     ap.add_argument("--probe-set-scene", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--probe-workload", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "cuda" else max(args.warmup, 1)
     select_workload(args.workload)
     if args.probe_set_scene:
@@ -675,6 +708,8 @@ def main():
     if fbf is not None:
         fbf_ms, fbf_rays = over_ranks([fbf[0]], MAX)[0], over_ranks([fbf[1]], SUM)[0]
     last_rays_all = over_ranks([last_frame_rays], SUM)[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gpu.read_accum(), gpu.read_img(), int(last_rays_all))
 
     # ---- N > 1: is the assembled multi-GPU frame the single-GPU frame, bit for bit? (rank 0 re-renders the same
     # frame ids on its own GPU alone: accum + img + ray count of the last frame) ----

@@ -81,20 +81,8 @@ int main(int argc, const char **argv)
         }
     }
 
-    // The reference looks for lib crt_<backend>.so next to the executable (util/render_plugin.cpp:7-18). This harness
-    // lives in oracle/_ref/ with the TEST plugins (oracle, embree, cuda_simt); the PRODUCT plugin libcrt_cuda.so is built
-    // into backends/cuda/_build/: when the requested plugin is not next to the harness but is there, point the
-    // (stand-in) SDL_GetBasePath at that directory.
-    if (!std::getenv("CRT_SDL_BASE_PATH")) {
-        char *base = SDL_GetBasePath();
-        const std::string here(base);
-        SDL_free(base);
-        const std::string lib = "libcrt_" + args[1] + ".so";
-        const std::string product_dir = here + "../../backends/cuda/_build/";
-        if (access((here + lib).c_str(), R_OK) != 0 && access((product_dir + lib).c_str(), R_OK) == 0) {
-            setenv("CRT_SDL_BASE_PATH", product_dir.c_str(), 1);
-        }
-    }
+    // The reference looks for lib crt_<backend>.so next to the executable (util/render_plugin.cpp:7-18): every plugin,
+    // the product's libcrt_cuda.so included, is built into oracle/_ref/ beside this harness.
     // main.cpp:65-66, :94-100
     auto plugin = std::make_unique<RenderPlugin>("crt_" + args[1]);
     ImGuiContext *ctx = ImGui::CreateContext();

@@ -92,20 +92,31 @@ def random_scene(rng):
                  samples_per_pixel=int(rng.integers(1, 4)))
 
 
-def one(seed):
+def case(seed):
+    """The random scene, framebuffer size, depth, frame count, camera and field of view of one seed."""
     rng = np.random.default_rng(seed)
     scene = random_scene(rng)
     w, h, depth, frames = int(rng.integers(8, 90)), int(rng.integers(8, 80)), int(rng.integers(1, 9)), int(rng.integers(1, 4))
     eye = rng.uniform(-9, 9, 3)
     cam = ArcballCamera(tuple(eye), tuple(rng.uniform(-1, 1, 3)), (0.0, 1.0, 0.0))
     fov = float(rng.uniform(20, 90))
-    ref, cpu = RefEmbreeBackend(max_depth=depth), OracleBackend(max_depth=depth)
-    for r in (ref, cpu):
-        r.initialize(w, h)
-        r.set_scene(scene)
+    return scene, w, h, depth, frames, cam, fov
+
+
+def render(backend, c):
+    """Renders case c on a fresh backend; returns it."""
+    scene, w, h, depth, frames, cam, fov = c
+    backend.initialize(w, h)
+    backend.set_scene(scene)
     for f in range(frames):
-        ref.render(cam.eye(), cam.dir(), cam.up(), fov, f == 0, True)
-        cpu.render(cam.eye(), cam.dir(), cam.up(), fov, f == 0, True)
+        backend.render(cam.eye(), cam.dir(), cam.up(), fov, f == 0, True)
+    return backend
+
+
+def one(seed):
+    c = case(seed)
+    scene, w, h, depth, frames = c[:5]
+    ref, cpu = render(RefEmbreeBackend(max_depth=depth), c), render(OracleBackend(max_depth=depth), c)
     a, b = ref.read_accum(), cpu.read_accum()
     same = np.array_equal(a.view(np.uint32), b.view(np.uint32)) or bool(((a == b) | (np.isnan(a) & np.isnan(b))).all())
     same_rays = np.array_equal(ref.read_ray_stats(), cpu.read_ray_stats())

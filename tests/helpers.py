@@ -1,5 +1,7 @@
-"""Shared test helpers: scenes, the host-check binding and the parity metric."""
+"""Shared test helpers: scenes, the host-check binding, the parity metric and the recorded results of the reference."""
 import ctypes as C
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -16,6 +18,40 @@ ABS_TOL = 1e-4
 REL_TOL = 1e-3
 MIN_MATCH_FRACTION = 0.999
 MAX_REL_L1 = 2e-3
+
+
+def digest(*arrays):
+    """Short fingerprint of arrays (dtype, shape and bytes): bit-exact comparison with a result stored as text."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f"{a.dtype.str}{a.shape}".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()[:16]
+
+
+def reference_result(table, key, compute=None):
+    """What the reference computed for `key`. compute() runs the reference's own code, where its binaries are built
+    (oracle/_ref/); pass None where they are not, and the result recorded in tests/golden/<table> is returned. A live result
+    must equal the recorded one, so that the table keeps what the reference computes. With CRT_RECORD_REFERENCE=1, every live
+    result is written into the table instead (how the table is regenerated)."""
+    path = os.path.join(ROOT, "tests", "golden", table)
+    recs = {}
+    if os.path.exists(path):
+        with open(path) as f:
+            recs = json.load(f)
+    if compute is None:
+        assert key in recs, f"{key}: no recorded result of the reference in tests/golden/{table} (the input has changed?)"
+        return recs[key]
+    rec = json.loads(json.dumps(compute()))  # (as stored: lists for tuples)
+    if os.environ.get("CRT_RECORD_REFERENCE") != "1":
+        assert key in recs, f"{key}: no recorded result of the reference in tests/golden/{table}; record it with CRT_RECORD_REFERENCE=1"
+        assert rec == recs[key], f"{key}: the reference's result differs from the one recorded in tests/golden/{table}"
+    else:
+        recs[key] = rec
+        with open(path, "w") as f:  # one record per line
+            f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(recs[k], separators=(',', ':'))}" for k in sorted(recs)) + "\n}\n")
+    return rec
 
 
 def parity(gpu_accum, ref_accum):

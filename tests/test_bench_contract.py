@@ -17,8 +17,8 @@ def _run(args, env=None, timeout=600):
                           env=e, timeout=timeout)
 
 
-def test_reference_arm_prints_one_json_line(built):
-    r = _run(["--impl", "reference", "--steps", "1", "--warmup", "0"])
+def test_reference_arm_prints_one_json_line(built, tmp_path):
+    r = _run(["--impl", "reference", "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path / "outputs")])
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1, r.stdout
@@ -32,6 +32,35 @@ def test_reference_arm_prints_one_json_line(built):
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+    import numpy as np
+
+    out = {p.stem: np.load(p) for p in (tmp_path / "outputs").glob("*.npy")}
+    assert sorted(out) == ["accum", "img", "num_rays"]
+    assert out["accum"].shape == (720, 1280, 3) and out["img"].shape == (720, 1280, 4) and out["num_rays"][0] > 0
+
+
+def test_dump_outputs_samples_a_large_frame_at_fixed_pixels(tmp_path):
+    """A frame over the size limit is written as the same seeded sample of pixels every time, with their indices."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    rng = np.random.default_rng(7)
+    accum = rng.normal(size=(30, 40, 3)).astype(np.float32)
+    img = rng.integers(0, 2 ** 32, size=(30, 40), dtype=np.uint64).astype(np.uint32)
+    limit = 4096 + 36 * 200  # 200 pixels of 12 + 16 bytes, plus an 8-byte index each
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), accum, img, 1234, limit=limit)
+    a, b = ({n: np.load(tmp_path / d / f"{n}.npy") for n in ("accum", "img", "num_rays", "pixel_index")} for d in ("a", "b"))
+    assert all(np.array_equal(a[n], b[n]) for n in a)
+    idx = a["pixel_index"].astype(np.int64)
+    assert a["pixel_index"].dtype == np.float64 and len(idx) == 200 and (np.diff(idx) > 0).all() and 0 <= idx[0] and idx[-1] < 30 * 40
+    assert a["accum"].dtype == np.float32 and np.array_equal(a["accum"], accum.reshape(-1, 3)[idx])
+    assert a["img"].dtype == np.float32 and np.array_equal(a["img"], img.view(np.uint8).reshape(-1, 4)[idx].astype(np.float32))
+    assert a["num_rays"].dtype == np.float64 and a["num_rays"].tolist() == [1234.0]
+    bench.dump_outputs(str(tmp_path / "whole"), accum, img, 1234)  # under the limit: the whole frame
+    assert np.array_equal(np.load(tmp_path / "whole" / "accum.npy"), accum) and not (tmp_path / "whole" / "pixel_index.npy").exists()
 
 
 def test_reference_arm_is_silent_on_other_ranks(built):
@@ -51,6 +80,11 @@ def test_gpu_arm_fails_loudly_without_a_gpu(built):
     assert "CUDA device" in r.stderr
 
 
+# Frames bench.py renders on its timed renderer with --steps 2 --warmup 3 and the default 5 repeats: 3 warm-up, 1 untimed
+# batch, 5 x 2 device-timed, 3 x 2 end-to-end.
+REPLAY_FRAMES = 3 + 1 + 5 * 2 + 3 * 2
+
+
 def test_gpu_arm_dry_run_on_the_emulated_renderer(built, tmp_path):
     """bench.py's GPU arm, every line of it — warm-up, the renderer's shadow-order decision, the counting pass, the
     untimed batch, the device-timed loop with frames in flight, the end-to-end loop, the CPU baseline, the JSON — run
@@ -63,7 +97,7 @@ def test_gpu_arm_dry_run_on_the_emulated_renderer(built, tmp_path):
     lib = simt_build.build()
     driver = tmp_path / "dry_run.py"
     driver.write_text(f'''
-import sys, time, types
+import os, sys, time, types
 sys.path.insert(0, {ROOT!r})
 import torch
 class _Stream:
@@ -87,9 +121,28 @@ backend._LIB_PATH, backend._lib = {lib!r}, None
 import bench
 sys.argv = ["bench.py"] + (sys.argv[1:] or ["--workload", "dev", "--steps", "2", "--warmup", "3"])
 bench.main()
+replay = os.environ.get("CRT_DRY_RUN_REPLAY")
+if replay and "--probe-set-scene" not in sys.argv and "--probe-workload" not in sys.argv:
+    # the same frames on a fresh renderer, one blocking call each: what the dumped outputs must be
+    import numpy as np
+    from chameleonrt_b200 import RenderCUDA
+    scene, view = bench.make_workload()
+    r = RenderCUDA(0, max_depth=bench.MAX_DEPTH)
+    r.initialize(bench.WIDTH, bench.HEIGHT)
+    r.set_scene(scene)
+    for f in range(int(replay.split(":")[0])):
+        st = r.render(*view, f == 0, True)
+    out = replay.split(":")[1]
+    os.makedirs(out)
+    np.save(out + "/accum.npy", r.read_accum())
+    np.save(out + "/img.npy", r.read_img())
+    np.save(out + "/num_rays.npy", np.array([st.num_rays], np.float64))
 ''')
-    r = subprocess.run([sys.executable, str(driver)], capture_output=True, text=True, cwd=ROOT, timeout=900,
-                       env=dict(os.environ, CRT_BENCH_REF_BUDGET="2", CRT_BENCH_PROBE_SCRIPT=str(driver)))
+    dump = tmp_path / "outputs"
+    r = subprocess.run([sys.executable, str(driver), "--workload", "dev", "--steps", "2", "--warmup", "3", "--dump-outputs", str(dump)],
+                       capture_output=True, text=True, cwd=ROOT, timeout=900,
+                       env=dict(os.environ, CRT_BENCH_REF_BUDGET="2", CRT_BENCH_PROBE_SCRIPT=str(driver),
+                                CRT_DRY_RUN_REPLAY=f"{REPLAY_FRAMES}:{tmp_path / 'replay'}"))
     assert r.returncode == 0, r.stderr[-3000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1, r.stdout
@@ -117,6 +170,19 @@ bench.main()
     assert "error" not in ss, ss
     assert ss["frames_bit_identical"] is True and ss["triangles"] == 34
     assert ss["host"]["set_scene_ms"] > 0 and ss["device"]["bvh8_nodes"] >= 1 and ss["device"]["closest_nodes_per_ray"] > 0
+    # --dump-outputs: the last timed step's framebuffers and ray count
+    import numpy as np
+
+    out = {p.stem: np.load(p) for p in dump.glob("*.npy")}
+    assert sorted(out) == ["accum", "img", "num_rays"]
+    assert out["accum"].dtype == np.float32 and out["accum"].shape == (48, 128, 3) and np.isfinite(out["accum"]).all()
+    assert out["img"].dtype == np.float32 and out["img"].shape == (48, 128, 4) and out["img"].max() <= 255 and out["img"].max() > 0
+    assert out["num_rays"].dtype == np.float64 and out["num_rays"].shape == (1,) and out["num_rays"][0] > 0
+    # ... and they are the last timed frame's: the same frames rendered again one by one give the same bits
+    replay = {n: np.load(tmp_path / "replay" / f"{n}.npy") for n in ("accum", "img", "num_rays")}
+    assert np.array_equal(out["accum"].view(np.uint32), replay["accum"].view(np.uint32))
+    assert np.array_equal(out["img"], replay["img"].view(np.uint8).reshape(48, 128, 4).astype(np.float32))
+    assert out["num_rays"].tolist() == replay["num_rays"].tolist()
 
 
 def test_gpu_arm_dry_run_two_ranks(built, tmp_path):
